@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference-side CPU path, same metric / config
+    python bench.py ... --dump-outputs DIR    # also save the last timed step's qpos as DIR/qpos.npy (seeded inputs)
 
 Headline (BASELINE.json metric: "hand-frames/sec (21-kpt -> Allegro 16-DoF), batch 65536"): VectorOptimizer, Allegro
 right hand, the shipped teleop config (scaling 1.6, huber 0.02, norm_delta 4e-3), one step = one batch of 65 536 synthetic
@@ -272,6 +273,8 @@ def main():
     ap.add_argument("--frames", type=int, default=FRAMES_PER_GPU, help="frames per GPU per step (headline)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="headline only (skip the per-configuration records)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the qpos the last timed headline step computed to DIR/qpos.npy "
+                    "(float32 [frames, 16]; qpos_rank<r>.npy per rank when several GPUs run), to compare two builds output for output")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -368,6 +371,10 @@ def main():
         barrier()
     total_ms = evs[0].elapsed_time(evs[-1])
     launch_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
+    if args.dump_outputs:  # `out` is reused by every later arm: save the last timed step's answers now
+        dump = Path(args.dump_outputs)
+        dump.mkdir(parents=True, exist_ok=True)
+        np.save(dump / ("qpos.npy" if world == 1 else f"qpos_rank{rank}.npy"), out.cpu().numpy())
 
     # ---- sustained: the same launch looped for >= 1 s ---------------------------------------------
     n_sus = max(args.steps, int(math.ceil(1.1e3 / max(statistics.mean(launch_ms), 1e-3))))

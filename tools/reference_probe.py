@@ -1,5 +1,5 @@
 """Is the REAL reference stack importable on this box?  pinocchio (pin>=3.3.1) + nlopt (nlopt>=2.8.0) + the reference package
-(baseline/_ref, DEX_RETARGETING_REFERENCE, /root/reference/src or site-packages).  Used by tests/test_real_reference.py and by
+(baseline/_ref, the source directory named by DEX_RETARGETING_REFERENCE, or site-packages).  Used by tests/test_real_reference.py and by
 `bench.py --impl reference`, which prefers the real thing (`kind: "reference"`) over the oracle's restated path (`"port"`)."""
 import importlib
 import os
@@ -19,7 +19,7 @@ def probe():
             found[name] = None
     found["reference"] = None
     if found["pinocchio"] and found["nlopt"]:
-        for cand in (os.environ.get("DEX_RETARGETING_REFERENCE"), ROOT / "baseline" / "_ref", "/root/reference/src", None):
+        for cand in (os.environ.get("DEX_RETARGETING_REFERENCE"), ROOT / "baseline" / "_ref", None):
             if cand is not None and not (Path(cand) / "dex_retargeting").exists():
                 continue
             if cand is not None:
