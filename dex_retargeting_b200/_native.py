@@ -89,6 +89,26 @@ EXPORTS = [
 ]
 
 _LIB = None
+_GRAD = None
+
+# The backward pass lives in a second library (include/dexr_grad.h); its exports are kept apart from EXPORTS, which mirrors dexr.h.
+GRAD_EXPORTS = ["dexr_grad_version", "dexr_grad_build_id", "dexr_grad_last_error", "dexr_grad_frames_sizeof", "dexr_grad_frames"]
+
+GRAD_STATUS_ACTIVE = 1 << 0
+GRAD_STATUS_SHIFTED = 1 << 1
+GRAD_STATUS_SINGULAR = 1 << 2
+GRAD_STATUS_SKIPPED = 1 << 3
+GRAD_STATUS_NONFINITE = 1 << 4
+
+
+class DexrGradFrames(C.Structure):
+    """Mirror of `dexr_grad_frames_t` (include/dexr_grad.h)."""
+
+    _fields_ = [
+        ("keypoints", C.c_void_p), ("ref_value", C.c_void_p), ("fixed_qpos", C.c_void_p), ("last_qpos", C.c_void_p),
+        ("projected", C.c_void_p), ("qpos", C.c_void_p), ("status", C.c_void_p), ("grad_qpos", C.c_void_p),
+        ("grad_keypoints", C.c_void_p), ("grad_ref_value", C.c_void_p), ("grad_last_qpos", C.c_void_p), ("grad_status", C.c_void_p),
+    ]
 
 
 def library_path() -> Path:
@@ -147,6 +167,39 @@ def load():
     # the single-robot entry points still work with it; dexr_solve_frames_multi, whose groups embed the struct, does not)
     _LIB = lib
     return lib
+
+
+def grad_library_path() -> Path:
+    return Path(__file__).resolve().parent / "libdexr_grad.so"
+
+
+def load_grad():
+    """Load libdexr_grad.so once (lazily: only the backward pass needs it); raise if it is missing or its layout disagrees."""
+    global _GRAD
+    if _GRAD is not None:
+        return _GRAD
+    path = grad_library_path()
+    if not path.exists():
+        raise DexrError(f"{path} not found: build the CUDA libraries first (python -c 'import __graft_entry__ as g; g.build()' "
+                        f"or python -m dex_retargeting_b200.build).  There is no CPU fallback.")
+    lib = C.CDLL(str(path))
+    lib.dexr_grad_version.restype = C.c_int
+    lib.dexr_grad_build_id.restype = C.c_char_p
+    lib.dexr_grad_last_error.restype = C.c_char_p
+    lib.dexr_grad_frames_sizeof.restype = C.c_size_t
+    lib.dexr_grad_frames.argtypes = [C.POINTER(DexrTable), C.c_void_p, C.POINTER(DexrParams), C.POINTER(DexrGradFrames), C.c_int64,
+                                     C.c_int, C.c_void_p]
+    if lib.dexr_grad_frames_sizeof() != C.sizeof(DexrGradFrames):
+        raise DexrError(f"dexr_grad_frames_t layout mismatch: library {lib.dexr_grad_frames_sizeof()} vs binding "
+                        f"{C.sizeof(DexrGradFrames)}")
+    _GRAD = lib
+    return lib
+
+
+def check_grad(code: int, what: str):
+    if code != 0:
+        msg = load_grad().dexr_grad_last_error().decode("utf-8", "replace")
+        raise DexrError(f"{what} failed ({code}): {msg}")
 
 
 def build_id() -> str:

@@ -65,8 +65,44 @@ def build_library(force: bool = False, verbose: bool = True, variant: str = "") 
     return out
 
 
+# The backward pass (include/dexr_grad.h) is a second library: libdexr.so stays the binary its build id and profiles name.
+GRAD_SRC = PKG / "csrc" / "dexr_grad.cu"
+GRAD_DEPS = [GRAD_SRC, PKG / "csrc" / "dexr_grad_kernels.cuh", PKG / "csrc" / "dexr_kernels.cuh",
+             PKG.parent / "include" / "dexr_grad.h", PKG.parent / "include" / "dexr.h"]
+GRAD_OUT = PKG / "libdexr_grad.so"
+
+
+def grad_source_id() -> str:
+    """16 hex digits over the backward library's sources and the headers they include (what `dexr_grad_build_id()` returns)."""
+    h = hashlib.sha256()
+    for d in GRAD_DEPS:
+        h.update(d.read_bytes())
+    return h.hexdigest()[:16]
+
+
+def build_grad_library(force: bool = False, verbose: bool = True) -> Path:
+    log_path = PKG / "csrc" / "build_grad.log"
+    if not force and GRAD_OUT.exists() and all(GRAD_OUT.stat().st_mtime >= d.stat().st_mtime for d in GRAD_DEPS):
+        return GRAD_OUT
+    cmd = [find_nvcc(), *NVCC_FLAGS, f'-DDEXR_GRAD_BUILD_ID="{grad_source_id()}"', "-o", str(GRAD_OUT), str(GRAD_SRC)]
+    if verbose:
+        print(" ".join(cmd), flush=True)
+    res = subprocess.run(cmd, capture_output=True, text=True)
+    log = (res.stdout or "") + (res.stderr or "")
+    log_path.write_text(log)
+    if res.returncode != 0:
+        sys.stderr.write(log)
+        raise RuntimeError(f"nvcc failed building {GRAD_OUT.name}")
+    if verbose:
+        for line in log.splitlines():
+            if "registers" in line or "spill" in line or "Compiling entry" in line:
+                print(line)
+    return GRAD_OUT
+
+
 if __name__ == "__main__":
     build_library(force="--force" in sys.argv)
+    build_grad_library(force="--force" in sys.argv)
     if "--variants" in sys.argv:
         for name in VARIANTS:
             build_library(force="--force" in sys.argv, variant=name)

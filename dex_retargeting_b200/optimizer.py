@@ -93,6 +93,7 @@ class Optimizer:
         self.opt_dof = len(idx_pin2target)  # includes nothing but the optimised joints
         self.opt = _SolverStats()
         self.last_status = None  # int32 status words of the most recent host-path solve (iterations | flags)
+        self.last_grad_status = None  # int32 DEXR_GRAD_STATUS_* words of the most recent retarget_batch backward pass
 
         self.target_link_human_indices = target_link_human_indices
         self.has_free_joint = len([n for n in robot.link_names if "dummy" in n]) >= 6
@@ -336,7 +337,28 @@ class Optimizer:
         rotation of the reference's detector are applied inside the solver (see `params`).
         `damping` [B] float32, in/out: the carried damping of B STREAMS that are fed frame by frame through this call
         (`StreamState.damping`, `dexr_frames_t.damping_io`); omit for independent frames.
-        Returns qpos [B,opt_dof] (= `out` if given).  Nothing is synchronised."""
+        Returns qpos [B,opt_dof] (= `out` if given).  Nothing is synchronised.
+        Autograd: when grad mode is on and `keypoints`, `ref_value` or `last_qpos` requires grad, the result carries a `grad_fn`
+        whose backward is the implicit-function gradient of each frame's minimiser (dex_retargeting_b200/grad.py; the forward
+        results are the same bits).  That route refuses `out=`, `raw_hand` and a `fixed_qpos` that requires grad; the per-frame
+        status of the last backward pass is left in `last_grad_status`."""
+        import torch
+
+        if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (keypoints, ref_value, last_qpos)):
+            from .grad import retarget_batch_autograd
+
+            return retarget_batch_autograd(self, keypoints=keypoints, ref_value=ref_value, last_qpos=last_qpos,
+                                           fixed_qpos=fixed_qpos, projected=projected, out=out, robot_qpos_out=robot_qpos_out,
+                                           status_out=status_out, cost_out=cost_out, clip_init=clip_init, stream=stream,
+                                           raw_hand=raw_hand, damping=damping)
+        return self._retarget_batch_launch(ref_value, fixed_qpos, last_qpos, keypoints=keypoints, projected=projected, out=out,
+                                           robot_qpos_out=robot_qpos_out, status_out=status_out, cost_out=cost_out,
+                                           clip_init=clip_init, stream=stream, raw_hand=raw_hand, damping=damping)
+
+    def _retarget_batch_launch(self, ref_value=None, fixed_qpos=None, last_qpos=None, *, keypoints=None, projected=None, out=None,
+                               robot_qpos_out=None, status_out=None, cost_out=None, clip_init=False, stream=None, raw_hand=None,
+                               damping=None):
+        """The one `dexr_solve_frames` launch behind `retarget_batch` (no autograd)."""
         import torch
 
         eng, io, p, out, B = self._prepare_batch(ref_value, fixed_qpos, last_qpos, keypoints=keypoints, projected=projected, out=out,
