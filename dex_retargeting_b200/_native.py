@@ -92,7 +92,8 @@ _LIB = None
 _GRAD = None
 
 # The backward pass lives in a second library (include/dexr_grad.h); its exports are kept apart from EXPORTS, which mirrors dexr.h.
-GRAD_EXPORTS = ["dexr_grad_version", "dexr_grad_build_id", "dexr_grad_last_error", "dexr_grad_frames_sizeof", "dexr_grad_frames"]
+GRAD_EXPORTS = ["dexr_grad_version", "dexr_grad_build_id", "dexr_grad_last_error", "dexr_grad_frames_sizeof", "dexr_grad_frames",
+                "dexr_grad_sequences_sizeof", "dexr_grad_sequences", "dexr_grad_lowpass"]
 
 GRAD_STATUS_ACTIVE = 1 << 0
 GRAD_STATUS_SHIFTED = 1 << 1
@@ -108,6 +109,18 @@ class DexrGradFrames(C.Structure):
         ("keypoints", C.c_void_p), ("ref_value", C.c_void_p), ("fixed_qpos", C.c_void_p), ("last_qpos", C.c_void_p),
         ("projected", C.c_void_p), ("qpos", C.c_void_p), ("status", C.c_void_p), ("grad_qpos", C.c_void_p),
         ("grad_keypoints", C.c_void_p), ("grad_ref_value", C.c_void_p), ("grad_last_qpos", C.c_void_p), ("grad_status", C.c_void_p),
+    ]
+
+
+class DexrGradSequences(C.Structure):
+    """Mirror of `dexr_grad_sequences_t` (include/dexr_grad.h)."""
+
+    _fields_ = [
+        ("keypoints", C.c_void_p), ("fixed_qpos", C.c_void_p), ("last_qpos", C.c_void_p), ("projected", C.c_void_p),
+        ("filter_init", C.c_void_p), ("qpos", C.c_void_p), ("status", C.c_void_p), ("grad_robot_qpos", C.c_void_p),
+        ("grad_last_qpos_out", C.c_void_p), ("grad_filter_state_out", C.c_void_p), ("projected_ws", C.c_void_p),
+        ("grad_keypoints", C.c_void_p), ("grad_last_qpos", C.c_void_p), ("grad_filter_state", C.c_void_p),
+        ("grad_status", C.c_void_p),
     ]
 
 
@@ -189,9 +202,17 @@ def load_grad():
     lib.dexr_grad_frames_sizeof.restype = C.c_size_t
     lib.dexr_grad_frames.argtypes = [C.POINTER(DexrTable), C.c_void_p, C.POINTER(DexrParams), C.POINTER(DexrGradFrames), C.c_int64,
                                      C.c_int, C.c_void_p]
+    lib.dexr_grad_sequences_sizeof.restype = C.c_size_t
+    lib.dexr_grad_sequences.argtypes = [C.POINTER(DexrTable), C.c_void_p, C.POINTER(DexrParams), C.POINTER(DexrGradSequences),
+                                        C.c_int64, C.c_int64, C.c_int, C.c_void_p]
+    lib.dexr_grad_lowpass.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int64, C.c_int64, C.c_int,
+                                      C.c_int, C.c_void_p]
     if lib.dexr_grad_frames_sizeof() != C.sizeof(DexrGradFrames):
         raise DexrError(f"dexr_grad_frames_t layout mismatch: library {lib.dexr_grad_frames_sizeof()} vs binding "
                         f"{C.sizeof(DexrGradFrames)}")
+    if lib.dexr_grad_sequences_sizeof() != C.sizeof(DexrGradSequences):
+        raise DexrError(f"dexr_grad_sequences_t layout mismatch: library {lib.dexr_grad_sequences_sizeof()} vs binding "
+                        f"{C.sizeof(DexrGradSequences)}")
     _GRAD = lib
     return lib
 

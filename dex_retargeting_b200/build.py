@@ -67,8 +67,8 @@ def build_library(force: bool = False, verbose: bool = True, variant: str = "") 
 
 # The backward pass (include/dexr_grad.h) is a second library: libdexr.so stays the binary its build id and profiles name.
 GRAD_SRC = PKG / "csrc" / "dexr_grad.cu"
-GRAD_DEPS = [GRAD_SRC, PKG / "csrc" / "dexr_grad_kernels.cuh", PKG / "csrc" / "dexr_kernels.cuh",
-             PKG.parent / "include" / "dexr_grad.h", PKG.parent / "include" / "dexr.h"]
+GRAD_DEPS = [GRAD_SRC, PKG / "csrc" / "dexr_grad_kernels.cuh", PKG / "csrc" / "dexr_grad_seq_kernels.cuh",
+             PKG / "csrc" / "dexr_kernels.cuh", PKG.parent / "include" / "dexr_grad.h", PKG.parent / "include" / "dexr.h"]
 GRAD_OUT = PKG / "libdexr_grad.so"
 
 

@@ -110,6 +110,7 @@ class SeqRetargeting:
         self.num_retargeting = 0
         self.filter = lp_filter
         self.is_warm_started = False
+        self.last_grad_status = None  # int32 [S,T] DEXR_GRAD_STATUS_* words of the most recent retarget_sequences backward pass
 
     # ------------------------------------------------------------------------------ single stream
     def warm_start(self, wrist_pos: np.ndarray, wrist_quat: np.ndarray, hand_type: HandType = HandType.right,
@@ -256,17 +257,48 @@ class SeqRetargeting:
         through T SeqRetargeting.retarget() steps in one launch.  Returns (robot_qpos [S,T,dof] float32
         in pinocchio joint order, filtered; state) -- `state` is updated in place and can be passed
         to the next call to continue the streams.  `raw_hand` (HandType): the keypoints are raw detector landmarks of that
-        hand, pre-processed inside the kernel (Optimizer.params)."""
+        hand, pre-processed inside the kernel (Optimizer.params).
+
+        Autograd: when grad mode is on and `keypoints`, `state.last_qpos` or `state.filter_state` requires grad, the result
+        carries a `grad_fn` whose backward walks every stream back in time (dex_retargeting_b200/grad.py: the implicit gradient
+        of each step's minimiser, chained through the warm-start anchor, the mimic fold and the low-pass filter).  The forward
+        results and exit state are the same bits as without autograd.  On that route `state.last_qpos` and
+        `state.filter_state` are REBOUND to new tensors (the exit state, part of the graph) instead of being written in place,
+        so a state passed to the next call carries the graph through the whole video, and `.detach()` on them truncates it;
+        `filter_init`, `projected` and `damping` are still updated in place.  The route refuses `out=`, `raw_hand` and a
+        `fixed_qpos` that requires grad; the [S,T] status words of the last backward pass are left in `last_grad_status`."""
         import torch
 
-        opt = self.optimizer
-        eng = opt.engine()
-        dev = torch.device("cuda", eng.device)
         if keypoints.dim() != 4 or tuple(keypoints.shape[2:]) != (N.NUM_KEYPOINTS, 3):
             raise ValueError(f"keypoints must have shape [S,T,21,3], got {tuple(keypoints.shape)}")
         S, T = int(keypoints.shape[0]), int(keypoints.shape[1])
         if state is None:
             state = self.make_stream_state(S)
+        if torch.is_grad_enabled() and any(t is not None and t.requires_grad
+                                           for t in (keypoints, state.last_qpos, state.filter_state)):
+            from .grad import retarget_sequences_autograd
+
+            return retarget_sequences_autograd(self, keypoints, state, fixed_qpos=fixed_qpos, out=out, status_out=status_out,
+                                               stream=stream, raw_hand=raw_hand)
+        dev = torch.device("cuda", self.optimizer.device_index)
+        if out is None:
+            out = torch.empty((S, T, self.optimizer.robot.dof), dtype=torch.float32, device=dev)
+        self._launch_sequences(keypoints, state, fixed_qpos, out, status_out, stream, lp_alpha=self.low_pass_alpha,
+                               raw_hand=raw_hand)
+        return out, state
+
+    def _launch_sequences(self, keypoints, state, fixed_qpos, out, status_out, stream, lp_alpha, raw_hand=None, last_qpos=None,
+                          filter_state=None):
+        """The one `dexr_solve_sequences` launch.  `last_qpos` / `filter_state`: the state buffers written in place (default:
+        the state's own)."""
+        import torch
+
+        opt = self.optimizer
+        eng = opt.engine()
+        dev = torch.device("cuda", eng.device)
+        S, T = int(keypoints.shape[0]), int(keypoints.shape[1])
+        last_qpos = state.last_qpos if last_qpos is None else last_qpos
+        filter_state = state.filter_state if filter_state is None else filter_state
 
         def chk(t, shape, dtype, name):
             if t.device != dev or t.dtype != dtype or not t.is_contiguous() or tuple(t.shape) != tuple(shape):
@@ -281,20 +313,17 @@ class SeqRetargeting:
             if fixed_qpos is None:
                 raise ValueError(f"Optimizer has {nf} joints but no fixed_qpos is given")
             io.fixed_qpos = chk(fixed_qpos, (S, T, nf), torch.float32, "fixed_qpos")
-        io.last_qpos = chk(state.last_qpos, (S, opt.opt_dof), torch.float32, "state.last_qpos")
-        io.filter_state = chk(state.filter_state, (S, opt.robot.dof), torch.float32, "state.filter_state")
+        io.last_qpos = chk(last_qpos, (S, opt.opt_dof), torch.float32, "state.last_qpos")
+        io.filter_state = chk(filter_state, (S, opt.robot.dof), torch.float32, "state.filter_state")
         io.filter_init = chk(state.filter_init, (S,), torch.uint8, "state.filter_init")
         if state.projected is not None:
             io.projected = chk(state.projected, (S, state.projected.shape[1]), torch.uint8, "state.projected")
         if state.damping is not None:
             io.damping_state = chk(state.damping, (S,), torch.float32, "state.damping")
-        if out is None:
-            out = torch.empty((S, T, opt.robot.dof), dtype=torch.float32, device=dev)
         io.robot_qpos_out = chk(out, (S, T, opt.robot.dof), torch.float32, "out")
         if status_out is not None:
             io.status_out = chk(status_out, (S, T), torch.int32, "status_out")
         s = stream if stream is not None else torch.cuda.current_stream(dev)
-        p = opt.params(clip_init=True, lp_alpha=self.low_pass_alpha, raw_hand=raw_hand)
+        p = opt.params(clip_init=True, lp_alpha=lp_alpha, raw_hand=raw_hand)
         N.check(eng.lib.dexr_solve_sequences(eng.handle, C.byref(p), C.byref(io), S, T, C.c_void_p(s.cuda_stream)),
                 "dexr_solve_sequences")
-        return out, state
